@@ -3,6 +3,7 @@
 bench.py -- the FFTPower hot path on synthetic log-normal particles.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME] [--order sorted|random]
+                  [--dump-outputs DIR]
 
 One "step" = one full FFTPower(...) / ConvolvedFFTPower(...) call on already-materialised particle columns:
 paint -> r2c -> compensate -> |delta(k)|^2 V -> binning -> BinnedStatistic on the host.
@@ -195,6 +196,32 @@ def result_arrays(r, cfg):
     return np.asarray(r.power['modes']), np.asarray(r.power['power'])
 
 
+def dump_outputs(r, directory):
+    """what a caller of the timed path receives, as DIR/<name>.npy: every column and the bin edges of the result's
+    BinnedStatistics (power, poles) and its non-empty numeric attrs.  Complex columns are split into <name>.real / <name>.imag;
+    float32 stays float32, everything else (integer mode counts included, exact below 2**53) becomes float64."""
+    os.makedirs(directory, exist_ok=True)
+    out = {}
+    for which in ("power", "poles"):
+        stat = getattr(r, which, None)
+        if stat is None:
+            continue
+        for v in stat.variables:
+            a = np.asarray(stat[v])
+            if np.iscomplexobj(a):
+                out["%s.%s.real" % (which, v)], out["%s.%s.imag" % (which, v)] = a.real, a.imag
+            else:
+                out["%s.%s" % (which, v)] = a
+        for d in stat.dims:
+            out["%s.edges.%s" % (which, d)] = stat.edges[d]
+    for k, v in r.attrs.items():
+        a = np.asarray(v)
+        if a.dtype.kind in "iuf" and a.size:        # numbers only; an empty setting (poles=[]) is no output
+            out["attrs.%s" % k] = a
+    for name, a in out.items():
+        np.save(os.path.join(directory, name + ".npy"), a.astype(np.float32 if a.dtype == np.float32 else np.float64))
+
+
 def compare(a, b, tol):
     ma, pa = a
     mb, pb = b
@@ -288,6 +315,8 @@ def run_ours(args):
         dist.all_reduce(tms, op=dist.ReduceOp.MAX)
     ms_step = float(tms.item()) / args.steps
     res_timed = result_arrays(r, cfg)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(r, args.dump_outputs)
 
     # ---- e2e: same call, columns start in pinned host memory
     def pinned(t):
@@ -596,7 +625,12 @@ def main():
     ap.add_argument("--npart", type=float, default=None, help="override the particle count (scratch runs)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-parity", action="store_true", help="skip the parity self-check")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step as DIR/<name>.npy (inputs are seeded: two builds "
+                         "run with the same arguments can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         # all host threads, also under torchrun (which exports OMP_NUM_THREADS=1); must precede the first OpenMP load
         os.environ["OMP_NUM_THREADS"] = str(os.cpu_count() or 1)

@@ -10,9 +10,14 @@ Generates the golden vectors under tests/golden/ by running the REFERENCE's own 
   mpirng.npz             : MPIRandomState streams (uniform / normal / poisson) + UniformCatalog N
   dataset_2d_modes.json  : sum over mu of `modes` in nbodykit/tests/data/dataset_2d.json
   binned_statistic_state.json : BinnedStatistic.__getstate__ of reference objects after slicing/reindexing
+  dataset_2d.json        : nbodykit/tests/data/dataset_2d.json, copied verbatim (a result file the reference wrote)
+  oracle_vs_reference.npz : the reference's outputs for the cases of tests/test_oracle_vs_reference.py; the long
+                           random streams are stored as a SHA-256 digest of their bytes plus 257 evenly spaced rows
 """
+import hashlib
 import json
 import os
+import shutil
 import sys
 
 import numpy as np
@@ -86,7 +91,9 @@ def golden_mpirng():
 
 
 def golden_dataset2d():
-    d = json.load(open(os.path.join(refload.REF, "nbodykit/tests/data/dataset_2d.json")))
+    src = os.path.join(refload.REF, "nbodykit/tests/data/dataset_2d.json")
+    shutil.copyfile(src, os.path.join(HERE, "dataset_2d.json"))
+    d = json.load(open(src))
     dt = [tuple(x) for x in d["data"]["__dtype__"]]
     names = [x[0] for x in dt]
     modes = np.array([[rec[names.index("modes")] for rec in row] for row in d["data"]["__data__"]])
@@ -137,12 +144,74 @@ def golden_binned_statistic():
     json.dump(out, open(os.path.join(HERE, "binned_statistic_state.json"), "w"))
 
 
+# the cases of tests/test_oracle_vs_reference.py (same order as its parametrisation)
+PROJECT_CASES = [
+    ([16, 16, 16], [64.] * 3, "c16", "f4", 5, [0, 2, 4], [0, 0, 1]),
+    ([12, 8, 10], [100., 50., 70.], "c8", "f4", 3, [1, 2], [0, 1, 0]),
+    ([16, 16, 16], [100.] * 3, "c16", "f8", 4, [3], [0.6, 0.0, 0.8]),
+    ([8, 8, 8], [1.] * 3, "c16", "f4", 1, [], [0, 0, 1]),
+]
+
+
+def stream_digest(a):
+    """(sha256 of dtype, shape and bytes, 257 evenly spaced rows): an exact fingerprint of an array too large to store"""
+    a = np.ascontiguousarray(a)
+    h = hashlib.sha256(("%s%s" % (a.dtype.str, a.shape)).encode())
+    h.update(a.tobytes())
+    return h.hexdigest(), a[np.linspace(0, len(a) - 1, 257).astype("i8")]
+
+
+def golden_oracle_vs_reference():
+    out = {}
+    for i, (N, L, cd, coord, Nmu, poles, los) in enumerate(PROJECT_CASES):
+        rng = np.random.RandomState(3)
+        shape = (N[0], N[1], N[2] // 2 + 1)
+        y = (rng.standard_normal(shape) + 1j * rng.standard_normal(shape)).astype(cd)
+        x = po.k_coords(N, L, coord)
+        dk = 2 * np.pi / min(L)
+        kedges = np.arange(0., np.pi * min(N) / max(L) + dk / 2, dk)
+        muedges = np.linspace(-1, 1, Nmu + 1)
+        res, pres = ns.project_to_basis(refload.RefComplexField(y, x), [kedges, muedges], los=los, poles=poles)
+        for j in range(4):
+            out["project%d_res%d" % (i, j)] = res[j]
+        if poles:
+            for j in range(3):
+                out["project%d_pole%d" % (i, j)] = pres[j]
+
+    N, L = [8, 16, 12], [10., 20., 30.]
+    rng = np.random.RandomState(4)
+    v = rng.standard_normal((8, 16, 7)) + 0j
+    for coord in ["f4", "f8"]:
+        w = po.k_coords(N, L, coord, kind="circular")
+        for interlaced in (True, False):
+            for res in ("cic", "tsc", "pcs"):
+                func = ns.get_compensation(interlaced, res)[0][1]
+                key = "comp_%s_%d_%s" % (coord, interlaced, res)
+                out[key + "_name"] = np.array(func.__name__)
+                out[key] = func(w, v.copy())
+
+    def stream(key, a):
+        digest, rows = stream_digest(a)
+        out[key + "_sha256"] = np.array(digest)
+        out[key + "_rows"] = rows
+
+    ref = ns.MPIRandomState(ns.FakeComm(), seed=7, size=123456)
+    stream("mpirng_uniform", ref.uniform(itemshape=(3,)))
+    stream("mpirng_normal", ref.normal())
+    ref = ns.MPIRandomState(ns.FakeComm(), seed=9, size=250001)
+    stream("product_uniform", ref.uniform(itemshape=(3,)))
+    stream("product_poisson", ref.poisson(lam=np.linspace(0.5, 3, 250001)))
+    stream("product_normal", ref.normal(loc=1., scale=3.))
+    np.savez_compressed(os.path.join(HERE, "oracle_vs_reference.npz"), **out)
+
+
 if __name__ == "__main__":
     golden_project()
     golden_compensate()
     golden_mpirng()
     golden_dataset2d()
     golden_binned_statistic()
+    golden_oracle_vs_reference()
     print("golden vectors written to", HERE)
 
 
