@@ -248,7 +248,8 @@ int nbk_ylm_mul_complex_acc2(void *acc, void *acc_mirror, const void *c, int dty
 /* Complex-dtype meshes (ParticleMesh(dtype='c16'/'c8'), base/mesh.py:50; convpower/catalog.py:151-176): pmesh keeps all
  * N^3 modes of the c2c transform.  The configuration-space fields of this path are real-valued, so the full spectrum
  * is the Hermitian completion of the r2c result: full[Nx][Ny][Nz] <- comp[Nx][Ny][Nz/2+1] (single GPU), and the
- * stored half is cut back out before a c2r (rows = planes * Ny of this rank). */
+ * stored half is cut back out before a c2r (rows = planes * Ny of this rank).  nbk_hermitian_expand takes power-of-two
+ * sides and the even 2^a 3^b 5^c 7^d sides of the mixed-radix transforms. */
 int nbk_hermitian_expand(const void *comp, void *full, int dtype, const int64_t *nmesh_host, void *stream);
 int nbk_hermitian_compress(const void *full, void *comp, int dtype, int64_t rows, int64_t Nz, void *stream);
 
@@ -266,6 +267,26 @@ int nbk_fft_lines_pack_range(const void *src, void *send, int dtype, int64_t n_l
                              int64_t o0, int64_t o_cnt, int P, int inverse, double scale, void *stream);
 int nbk_slab_push_range(const void *send, void *const *peer_ptrs_host, int dtype, int64_t rows_per_peer, int64_t n_outer,
                         int64_t n_inner, int64_t outer_start, int64_t o0, int64_t o_cnt, int P, int rank, void *stream);
+
+/* Mixed-radix transforms for mesh sides N = 2^a 3^b 5^c 7^d (meshes such as 384, 768, 1000, 1536 per side; pmesh/pfft
+ * transform any size, base/mesh.py:228,237).  Same layout, normalisation and precision as nbk_r2c / nbk_c2r and the line
+ * passes above; RealField.r2c / ComplexField.c2r call these only when a side is not a power of two.  They accept powers of
+ * two as well.  Every entry point validates before any CUDA call; sizes: lines 2 <= n_line <= 8192, any 7-smooth length
+ * (a line pass is complex-to-complex); z pass Nz even, 7-smooth, <= 16384; whole mesh every side even and 7-smooth,
+ * Nx, Ny <= 8192, Nz <= 16384.
+ *   nbk_fft_mr_lines : strided batched complex lines, element (outer, n, inner) at
+ *                      outer*outer_stride + n*line_stride + inner (the addressing of nbk_fft_lines); src == dst is in
+ *                      place; inverse != 0 is the unnormalised backward transform; the output is multiplied by scale.
+ *   nbk_fft_mr_z     : inverse == 0: real rows [rows][Nz] -> complex rows [rows][Nz/2+1]; inverse != 0: the reverse
+ *                      (unnormalised); times scale.  src and dst must be distinct buffers.
+ *   nbk_r2c_mr / nbk_c2r_mr : the single-GPU whole-mesh transforms, parameters as nbk_r2c / nbk_c2r (nbk_c2r_mr
+ *                      destroys its input unless `work`, the size of cplx, is given). */
+int nbk_fft_mr_lines(const void *src, void *dst, int dtype, int64_t n_line, int64_t line_stride, int64_t n_inner,
+                     int64_t n_outer, int64_t outer_stride, int inverse, double scale, void *stream);
+int nbk_fft_mr_z(const void *src, void *dst, int dtype, int64_t rows, int64_t Nz, int inverse, double scale,
+                 void *stream);
+int nbk_r2c_mr(const void *real, void *cplx, int dtype, const int64_t *nmesh_host, double extra_scale, void *stream);
+int nbk_c2r_mr(const void *cplx, void *real, int dtype, const int64_t *nmesh_host, void *work, void *stream);
 
 /* Fourier-space resampling to another mesh size: pmesh `Field.resample`, called by MeshSource.compute(Nmesh=...)
  * (base/mesh.py:317-327).  Modes both meshes represent are copied (same integer frequency label per axis, Nyquist

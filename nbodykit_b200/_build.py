@@ -18,6 +18,7 @@ SOURCES = [
     ("core.cu", []),
     ("paint.cu", ["--fmad=false"]),
     ("fft.cu", []),
+    ("fft_mixed.cu", []),
     ("binning.cu", ["--fmad=false"]),
     ("ylm.cu", []),
     ("route.cu", ["--fmad=false"]),
@@ -35,7 +36,8 @@ def _nvcc():
 
 def _stamp(path, flags):
     h = hashlib.sha1()
-    for dep in [path, os.path.join(CSRC, "common.cuh"), os.path.join(CSRC, "ylm_table.inc"),
+    for dep in [path, os.path.join(CSRC, "common.cuh"), os.path.join(CSRC, "fft_common.cuh"),
+                os.path.join(CSRC, "ylm_table.inc"),
                 os.path.join(HERE, "..", "include", "nbk_b200.h")]:
         with open(dep, "rb") as f:
             h.update(f.read())

@@ -49,6 +49,10 @@ SIGNATURES = {
     "nbk_fft_lines": ([_vp, _i, _i64, _i64, _i64, _i64, _i64, _i, _d, _vp], _i),
     "nbk_fft_lines_oop": ([_vp, _vp, _i, _i64, _i64, _i64, _i64, _i64, _i, _d, _vp], _i),
     "nbk_fft_z_forward": ([_vp, _vp, _i, _i64, _i64, _vp], _i),
+    "nbk_fft_mr_lines": ([_vp, _vp, _i, _i64, _i64, _i64, _i64, _i64, _i, _d, _vp], _i),
+    "nbk_fft_mr_z": ([_vp, _vp, _i, _i64, _i64, _i, _d, _vp], _i),
+    "nbk_r2c_mr": ([_vp, _vp, _i, _pi64, _d, _vp], _i),
+    "nbk_c2r_mr": ([_vp, _vp, _i, _pi64, _vp, _vp], _i),
     "nbk_fft_lines_scatter": ([_vp, ctypes.POINTER(ctypes.c_void_p), _i, _i64, _i64, _i64, _i64, _i, _i, _d, _vp], _i),
     "nbk_transpose_pack": ([_vp, _vp, _i, _i64, _i64, _i64, _i64, _vp], _i),
     "nbk_transpose_unpack": ([_vp, _vp, _i, _i64, _i64, _i64, _i64, _vp], _i),

@@ -15,26 +15,15 @@
 // global memory, last stage straight to the digit-reversed frequency rows, [N][B+1] padded tiles in between) and the
 // shared-memory kernels (k_fft_lines with cp.async double buffering, k_fft_z_r2c, k_fft_z_c2r).
 // Decimation-in-frequency radix-8 butterflies in registers throughout (+ one radix-4 / radix-2 stage for the remainder of
-// log2 N).  Twiddles: f8-accurate table built on the device with sincospi, staged in shared memory.  Sizes: 2^k.
-#include "common.cuh"
+// log2 N).  Twiddles: f8-accurate table built on the device with sincospi, staged in shared memory.  Sizes: 2^k (other
+// 2^a 3^b 5^c 7^d sizes: fft_mixed.cu).
+#include "fft_common.cuh"
 #include <cuda.h>      // CUtensorMap types only: the encoder comes from cudaGetDriverEntryPoint (no -lcuda)
 #include <map>
 #include <mutex>
 #include <tuple>
 #include <stdlib.h>
 #include <string.h>
-
-template <typename T> struct C2;
-template <> struct C2<float> { typedef float2 type; };
-template <> struct C2<double> { typedef double2 type; };
-
-template <typename C> __device__ __forceinline__ C cadd(C a, C b) { return C{a.x + b.x, a.y + b.y}; }
-template <typename C> __device__ __forceinline__ C csub(C a, C b) { return C{a.x - b.x, a.y - b.y}; }
-template <typename C> __device__ __forceinline__ C cmul(C a, C b) {
-    return C{a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x};
-}
-template <typename C> __device__ __forceinline__ C cconj(C a) { return C{a.x, -a.y}; }
-template <typename C> __device__ __forceinline__ C cmuli_neg(C a) { return C{a.y, -a.x}; }  // a * (-i)
 
 // Stage plan: radix-8 stages, then one radix-4 or radix-2 stage for the remainder of log2(N).
 // position (in the in-place DIF output) of frequency k = mixed-radix digit reversal
@@ -50,20 +39,6 @@ __device__ __forceinline__ int pos_of_freq(int k, int N, int log2n) {
     if (r == 2) pos += (rem & 3);        // base == 4 -> base/4 == 1
     else if (r == 1) pos += (rem & 1);
     return pos;
-}
-
-template <typename C> struct Sqrt1_2;
-template <> struct Sqrt1_2<float2> { static __device__ __forceinline__ float v() { return 0.70710678118654752440f; } };
-template <> struct Sqrt1_2<double2> { static __device__ __forceinline__ double v() { return 0.70710678118654752440; } };
-
-// 4-point DFT (forward): X0 = c0+c1, X1 = c2+c3, X2 = c0-c1, X3 = c2-c3
-template <typename C>
-__device__ __forceinline__ void dft4(C &a0, C &a1, C &a2, C &a3) {
-    C c0 = cadd(a0, a2), c1 = cadd(a1, a3), c2 = csub(a0, a2), c3 = cmuli_neg(csub(a1, a3));
-    a0 = cadd(c0, c1);
-    a1 = cadd(c2, c3);
-    a2 = csub(c0, c1);
-    a3 = csub(c2, c3);
 }
 
 // Shared-memory address (in elements) of line element e, column b.  Rows are padded to B+1 elements; with SKEW an
@@ -300,19 +275,6 @@ k_fft_lines_scatter(const typename C2<T>::type *__restrict__ src, PeerPtrs<typen
 // CTA, so 2-3 CTAs share an SM and one CTA's global phase overlaps another's butterflies.
 // PEER: the store goes to the NVLink-mapped transposed field of rank k / n_per (see k_fft_lines_scatter).
 // ---------------------------------------------------------------------------------------------
-template <typename C>
-__device__ __forceinline__ void radix8(C (&a)[8]) {   // in: a[j] = x_j ; out: a[m] = X_m (8-point forward DFT)
-    C b0 = cadd(a[0], a[4]), b1 = cadd(a[1], a[5]), b2 = cadd(a[2], a[6]), b3 = cadd(a[3], a[7]);
-    C b4 = csub(a[0], a[4]), d5 = csub(a[1], a[5]), d6 = csub(a[2], a[6]), d7 = csub(a[3], a[7]);
-    const auto h = Sqrt1_2<C>::v();
-    C b5 = C{(d5.x + d5.y) * h, (d5.y - d5.x) * h};
-    C b6 = cmuli_neg(d6);
-    C b7 = C{(d7.y - d7.x) * h, -(d7.x + d7.y) * h};
-    dft4(b0, b1, b2, b3);      // -> X0, X2, X4, X6
-    dft4(b4, b5, b6, b7);      // -> X1, X3, X5, X7
-    a[0] = b0; a[1] = b4; a[2] = b1; a[3] = b5; a[4] = b2; a[5] = b6; a[6] = b3; a[7] = b7;
-}
-
 __device__ __forceinline__ int rev8(int t, int ndig) {   // reverse the ndig base-8 digits of t
     int r = 0;
     for (int i = 0; i < ndig; i++) { r = (r << 3) | (t & 7); t >>= 3; }
@@ -836,11 +798,7 @@ k_fft_z_r2c(const T *__restrict__ real, typename C2<T>::type *__restrict__ cplx,
             if (b < bvalid) {
                 C zk = sm[saddr<B, true>(pos_of_freq(k & (M - 1), M, log2m), sk) + b];
                 C zm = cconj(sm[saddr<B, true>(pos_of_freq((M - k) & (M - 1), M, log2m), sk) + b]);
-                C e = cadd(zk, zm), o = csub(zk, zm);
-                C wo = cmul(twN[k], o);          // W_N^k (Z[k] - conj Z[M-k])
-                C x = C{e.x + wo.y, e.y - wo.x};  // e - i*wo
-                T h = (T)0.5 * scale;
-                dst[(int64_t)b * Nzc + k] = C{x.x * h, x.y * h};
+                dst[(int64_t)b * Nzc + k] = hermitian_split(zk, zm, twN[k], (T)0.5 * scale);
             }
         }
         __syncthreads();
@@ -1151,13 +1109,7 @@ k_fft_z_c2r(const typename C2<T>::type *__restrict__ cplx, T *__restrict__ real,
             int k = w & (M - 1), b = w >> log2m;
             C v = C{0, 0};
             if (b < bvalid) {
-                C xk = src[(int64_t)b * Nzc + k];
-                C xm = cconj(src[(int64_t)b * Nzc + (M - k)]);
-                C e = cadd(xk, xm), d = csub(xk, xm);
-                C o = cmul(cconj(twN[k]), d);
-                // Z = (e + i o)/2 ; the factor 2 of the unnormalised inverse cancels the 1/2
-                C z = C{e.x - o.y, e.y + o.x};
-                v = cconj(z);
+                v = hermitian_merge(src[(int64_t)b * Nzc + k], cconj(src[(int64_t)b * Nzc + (M - k)]), twN[k]);
             }
             sm[saddr<B, true>(k, sk) + b] = v;
         }
@@ -1192,7 +1144,7 @@ __global__ void k_twiddle(typename C2<T>::type *tw, int N) {
 static std::mutex g_tw_mutex;
 static std::map<std::tuple<int, int, int>, void *> g_tw;
 
-static int get_twiddle(int N, int dtype, cudaStream_t s, void **out) {
+int get_twiddle(int N, int dtype, cudaStream_t s, void **out) {
     int dev = 0;
     NBK_CUDA(cudaGetDevice(&dev));
     std::lock_guard<std::mutex> lock(g_tw_mutex);
@@ -1841,7 +1793,10 @@ k_hermitian_compress(const C *__restrict__ full, C *__restrict__ comp, int64_t r
 }
 
 extern "C" int nbk_hermitian_expand(const void *comp, void *full, int dtype, const int64_t *nmesh, void *stream) {
-    int rc = check_dims("hermitian_expand", dtype, nmesh[0], nmesh[1], nmesh[2]);
+    // power-of-two sides (the transform of nbk_r2c) or the even 7-smooth sides of the mixed-radix nbk_r2c_mr
+    int rc = (is_pow2(nmesh[0]) && is_pow2(nmesh[1]) && is_pow2(nmesh[2]))
+                 ? check_dims("hermitian_expand", dtype, nmesh[0], nmesh[1], nmesh[2])
+                 : nbk_check_mixed_dims("hermitian_expand", dtype, nmesh[0], nmesh[1], nmesh[2]);
     if (rc) return rc;
     NBK_CHECK_ARG(comp != nullptr && full != nullptr && comp != full, "hermitian_expand: needs two distinct buffers");
     int64_t rows = nmesh[0] * nmesh[1];

@@ -45,6 +45,10 @@ def _ptr(t):
     return ctypes.c_void_p(t.data_ptr() if t is not None else None)
 
 
+def _is_pow2(n):
+    return n > 0 and (n & (n - 1)) == 0
+
+
 def current_device():
     if not torch.cuda.is_available():
         raise _lib.NbkError("nbodykit_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
@@ -241,6 +245,9 @@ class ParticleMesh(object):
         self.y_start = self.comm.rank * self.y_n
         self.Nzc = Nz if self.cplx else Nz // 2 + 1      # stored length of the last axis of a ComplexField
         self.transposed = P > 1
+        # power-of-two meshes use the transform of fft.cu (NVLink peer transpose when P > 1); any other side goes
+        # through the mixed-radix transform of fft_mixed.cu (sides 2^a 3^b 5^c 7^d, every side even; others raise)
+        self.mixed_fft = not all(_is_pow2(n) for n in (Nx, Ny, Nz))
         self._nmesh_c = iarr(self.Nmesh)
         self._box_c = darr(self.BoxSize)
         self._coords = {}
@@ -883,12 +890,22 @@ class RealField(Field):
         if pm.cplx:
             half = torch.empty((Nx, Ny, Nz // 2 + 1), dtype=out.value.dtype, device=out.value.device)
             with stage("r2c"):
-                check(lib().nbk_r2c(_ptr(self.value), _ptr(half), code, pm._nmesh_c, float(scale), _stream()), "nbk_r2c")
+                if pm.mixed_fft:
+                    check(lib().nbk_r2c_mr(_ptr(self.value), _ptr(half), code, pm._nmesh_c, float(scale), _stream()),
+                          "nbk_r2c_mr")
+                else:
+                    check(lib().nbk_r2c(_ptr(self.value), _ptr(half), code, pm._nmesh_c, float(scale), _stream()), "nbk_r2c")
                 check(lib().nbk_hermitian_expand(_ptr(half), _ptr(out.value), code, pm._nmesh_c, _stream()),
                       "nbk_hermitian_expand")
+        elif P == 1 and pm.mixed_fft:
+            with stage("r2c"):
+                check(lib().nbk_r2c_mr(_ptr(self.value), _ptr(out.value), code, pm._nmesh_c, float(scale), _stream()),
+                      "nbk_r2c_mr")
         elif P == 1:
             with stage("r2c"):
                 check(lib().nbk_r2c(_ptr(self.value), _ptr(out.value), code, pm._nmesh_c, float(scale), _stream()), "nbk_r2c")
+        elif pm.mixed_fft:
+            self._r2c_mixed_slabs(out, float(scale))
         else:
             Nzc = pm.Nzc
             work = torch.empty((pm.x_n, Ny, Nzc), dtype=out.value.dtype, device=out.value.device)
@@ -964,6 +981,30 @@ class RealField(Field):
         out.attrs = dict(self.attrs)
         return out
 
+    def _r2c_mixed_slabs(self, out, scale):
+        """P > 1, mixed-radix sizes: z and y passes on the x slab, pack + NCCL all-to-all + unpack into the transposed
+        [y_n][Nx][Nzc] layout, x pass (the NVLink peer transpose serves power-of-two sizes only)"""
+        pm = self.pm
+        L, code, P = lib(), _CODE[pm.typestr], pm.comm.size
+        Nx, Ny, Nz = [int(v) for v in pm.Nmesh]
+        Nzc = pm.Nzc
+        work = torch.empty((pm.x_n, Ny, Nzc), dtype=out.value.dtype, device=out.value.device)
+        with stage("fft_zy"):
+            check(L.nbk_fft_mr_z(_ptr(self.value), _ptr(work), code, pm.x_n * Ny, Nz, 0, 1.0, _stream()), "fft_mr_z")
+            check(L.nbk_fft_mr_lines(_ptr(work), _ptr(work), code, Ny, Nzc, Nzc, pm.x_n, Ny * Nzc, 0, 1.0, _stream()),
+                  "fft_mr_lines(y)")
+        send = torch.empty_like(work)
+        with stage("fft_pack"):
+            check(L.nbk_transpose_pack(_ptr(work), _ptr(send), code, pm.x_n, Ny, Nzc, P, _stream()), "transpose_pack")
+        recv = torch.view_as_real(work).view(-1)
+        with stage("fft_alltoall"):
+            pm.comm.all_to_all_single(recv, torch.view_as_real(send).view(-1))
+        with stage("fft_unpack"):
+            check(L.nbk_transpose_unpack(_ptr(recv), _ptr(out.value), code, pm.y_n, Nx, Nzc, P, _stream()), "transpose_unpack")
+        with stage("fft_x"):
+            check(L.nbk_fft_mr_lines(_ptr(out.value), _ptr(out.value), code, Nx, Nzc, Nzc, pm.y_n, Nx * Nzc, 0,
+                                     scale / (float(Nx) * Ny * Nz), _stream()), "fft_mr_lines(x)")
+
 
 class BaseComplexField(Field):
     pass
@@ -1007,7 +1048,14 @@ class ComplexField(BaseComplexField):
             half = torch.empty((Nx, Ny, Nz // 2 + 1), dtype=self.value.dtype, device=self.value.device)
             check(lib().nbk_hermitian_compress(_ptr(self.value), _ptr(half), code, Nx * Ny, Nz, _stream()),
                   "nbk_hermitian_compress")
-            check(lib().nbk_c2r(_ptr(half), _ptr(out.value), code, pm._nmesh_c, None, _stream()), "nbk_c2r")
+            if pm.mixed_fft:
+                check(lib().nbk_c2r_mr(_ptr(half), _ptr(out.value), code, pm._nmesh_c, None, _stream()), "nbk_c2r_mr")
+            else:
+                check(lib().nbk_c2r(_ptr(half), _ptr(out.value), code, pm._nmesh_c, None, _stream()), "nbk_c2r")
+            out.attrs = dict(self.attrs)
+            return out
+        if pm.mixed_fft:
+            self._c2r_mixed(out)
             out.attrs = dict(self.attrs)
             return out
         st = pm._peer_stage() if P > 1 else None
@@ -1051,6 +1099,35 @@ class ComplexField(BaseComplexField):
             check(lib().nbk_fft_zy_backward(_ptr(slab), _ptr(out.value), code, pm.x_n, Ny, Nz, _stream()), "fft_zy_backward")
         out.attrs = dict(self.attrs)
         return out
+
+    def _c2r_mixed(self, out):
+        """the mixed-radix inverse: one GPU in one call; P > 1 mirrors _r2c_mixed_slabs (inverse x pass, pack back +
+        NCCL all-to-all + unpack back, inverse y and z passes on the x slab).  The complex field is only read."""
+        pm = self.pm
+        L, code, P = lib(), _CODE[pm.typestr], pm.comm.size
+        Nx, Ny, Nz = [int(v) for v in pm.Nmesh]
+        work = torch.empty_like(self.value)
+        if P == 1:
+            with stage("c2r"):
+                check(L.nbk_c2r_mr(_ptr(self.value), _ptr(out.value), code, pm._nmesh_c, _ptr(work), _stream()), "nbk_c2r_mr")
+            return
+        Nzc = pm.Nzc
+        with stage("ifft_x"):
+            check(L.nbk_fft_mr_lines(_ptr(self.value), _ptr(work), code, Nx, Nzc, Nzc, pm.y_n, Nx * Nzc, 1, 1.0, _stream()),
+                  "fft_mr_lines(x)")
+        send = torch.empty_like(work)
+        with stage("ifft_pack"):
+            check(L.nbk_transpose_pack_back(_ptr(work), _ptr(send), code, pm.y_n, Nx, Nzc, P, _stream()), "pack_back")
+        recv = torch.view_as_real(work).view(-1)
+        with stage("ifft_alltoall"):
+            pm.comm.all_to_all_single(recv, torch.view_as_real(send).view(-1))
+        slab = torch.view_as_real(send).view(-1)
+        with stage("ifft_unpack"):
+            check(L.nbk_transpose_unpack_back(_ptr(recv), _ptr(slab), code, pm.x_n, Ny, Nzc, P, _stream()), "unpack_back")
+        with stage("ifft_zy"):
+            check(L.nbk_fft_mr_lines(_ptr(slab), _ptr(slab), code, Ny, Nzc, Nzc, pm.x_n, Ny * Nzc, 1, 1.0, _stream()),
+                  "fft_mr_lines(y)")
+            check(L.nbk_fft_mr_z(_ptr(slab), _ptr(out.value), code, pm.x_n * Ny, Nz, 1, 1.0, _stream()), "fft_mr_z")
 
     def compensate(self, name):
         """v /= window transfer function (source/mesh/catalog.py:449-594), in place"""
