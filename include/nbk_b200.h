@@ -294,6 +294,54 @@ int nbk_c2r_mr(const void *cplx, void *real, int dtype, const int64_t *nmesh_hos
 int nbk_resample_complex(const void *src, void *dst, int dtype, const int64_t *nmesh_src_host,
                          const int64_t *nmesh_dst_host, void *stream);
 
+/* Friends-of-friends groups (FOF, algorithms/fof.py: kdcount `cluster.fof` in _fof_local :289-309, equiv_class :538-607,
+ * centerofmass :647-700).  Two rows are friends when their squared separation, evaluated in f64 from the stored
+ * positions, is <= ll^2; periodic calls use the minimum-image difference per axis (box_host = the three periods), a
+ * NULL box means non-periodic and then lo_host / hi_host (the data bounds) place the cell grid.  Positions are [n][3]
+ * rows of pos_dtype F4|F8, 0 <= n <= 2^31-1 (int32 union-find), ll > 0.  Every call checks its arguments before any
+ * CUDA call.  The call sequence is workspace -> bucket -> link -> compress -> minid:
+ *   nbk_fof_workspace : bytes of scratch the other calls need for this (n, ll, box | bounds); ncell_host (optional,
+ *                       host int64[3]) receives the cell grid: cells of side >= ll, at most max(27, 2n) of them (the
+ *                       side grows beyond ll when the cap binds).  Negative on a rejected argument.
+ *   nbk_fof_bucket    : counting sort of the rows by cell.  order: int32[n], row of every sorted slot (rows of one
+ *                       cell are adjacent, in no fixed order); spos: [3][n] of pos_dtype, the positions in that order
+ *                       (structure of arrays).  `work` keeps the cell starts for nbk_fof_link.
+ *   nbk_fof_link      : union-find over sorted slots: each slot visits the later slots of its own cell and the 13
+ *                       forward neighbour cells (neighbours that wrap onto the same cell are visited once).  parent:
+ *                       int32[n], written from scratch; afterwards it is a forest whose roots are the smallest slot of
+ *                       each group.  Same (dtype, n, ll, box, bounds, work) as the bucket call.
+ *   nbk_fof_compress  : root: int32[n] by ROW, root[order[i]] = root slot of slot i (parent is compressed in place).
+ *   nbk_fof_minid     : out[row] = min over the row's group of value[row] (value NULL: row_offset + row, the global
+ *                       row index -- the `minid` of _fof_local :302-307); rootmin: int64[n] scratch.  Called again with
+ *                       updated values it pushes a change to the whole local group (the merge of _fof_merge :311-337).
+ *   nbk_fof_reduce    : dense per-group reductions for find_features, group g = label[row] in [0, ngroups) (label
+ *                       int64[n], other values skipped).  Rows are visited as order[0..n_visit) (rows >= n skipped) or,
+ *                       with order NULL, 0..n.  val: [n][dim] of val_dtype (dim 1..3) or NULL (count only).  Outputs
+ *                       are ACCUMULATED into (initialise them first):
+ *                         op NBK_FOF_SUM : osum f64[ngroups][dim] += val, or += (val - anchor) wrapped into
+ *                                          [-L/2, L/2) on every axis when box_host is given (anchor:
+ *                                          int64[ngroups][dim] keys from op MIN); ocount uint64[ngroups] (optional)
+ *                                          += 1 per row.
+ *                         op NBK_FOF_MIN / NBK_FOF_MAX : okey int64[ngroups][dim] = min / max of the order-preserving
+ *                                          key of (double)val: bits b of the double, b >= 0 ? b : b ^ (2^63 - 1).
+ *                       peak / peakmax (f64[n] and int64 keys [ngroups]): a row whose peak value is below its
+ *                       group's peakmax counts for group 0 instead (fof_catalog's `label1` :510). */
+#define NBK_FOF_SUM 0
+#define NBK_FOF_MIN 1
+#define NBK_FOF_MAX 2
+int64_t nbk_fof_workspace(int64_t n, double ll, const double *box_host, const double *lo_host, const double *hi_host,
+                          int64_t *ncell_host);
+int nbk_fof_bucket(const void *pos, int pos_dtype, int64_t n, double ll, const double *box_host, const double *lo_host,
+                   const double *hi_host, void *work, int64_t work_bytes, int32_t *order, void *spos, void *stream);
+int nbk_fof_link(const void *spos, int pos_dtype, int64_t n, double ll, const double *box_host, const double *lo_host,
+                 const double *hi_host, const void *work, int64_t work_bytes, int32_t *parent, void *stream);
+int nbk_fof_compress(int32_t *parent, int64_t n, const int32_t *order, int32_t *root, void *stream);
+int nbk_fof_minid(const int32_t *root, int64_t n, const int64_t *value, int64_t row_offset, int64_t *rootmin,
+                  int64_t *out, void *stream);
+int nbk_fof_reduce(int op, const int64_t *label, int64_t n, const int32_t *order, int64_t n_visit, const void *val,
+                   int val_dtype, int dim, const int64_t *anchor, const double *box_host, const double *peak,
+                   const int64_t *peakmax, int64_t ngroups, double *osum, int64_t *okey, int64_t *ocount, void *stream);
+
 /* elementwise helpers behind RealField/ComplexField `[...] = v`, `*= a`, `+= other`
  * (source/mesh/catalog.py:203,354,396-398; fftpower.py:128).  n counts REAL scalars. */
 int nbk_fill(void *x, int dtype, int64_t n, double value, void *stream);

@@ -22,6 +22,7 @@ SOURCES = [
     ("binning.cu", ["--fmad=false"]),
     ("ylm.cu", []),
     ("route.cu", ["--fmad=false"]),
+    ("fof.cu", []),
 ]
 COMMON = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
           "-Xcompiler", "-fPIC", "-Xcompiler", "-O3"]

@@ -75,6 +75,12 @@ SIGNATURES = {
     "nbk_ylm_mul_real": ([_vp, _vp, _i, _i, _i, _pi64, _pd, _pd, _i64, _i64, _vp], _i),
     "nbk_ylm_mul_complex_acc": ([_vp, _vp, _i, _i, _i, _pi64, _pd, _i, _i64, _i64, _vp], _i),
     "nbk_cross_power": ([_vp, _vp, _vp, _i, _i64, _d, _i, _vp], _i),
+    "nbk_fof_workspace": ([_i64, _d, _pd, _pd, _pd, _pi64], _i64),
+    "nbk_fof_bucket": ([_vp, _i, _i64, _d, _pd, _pd, _pd, _vp, _i64, _vp, _vp, _vp], _i),
+    "nbk_fof_link": ([_vp, _i, _i64, _d, _pd, _pd, _pd, _vp, _i64, _vp, _vp], _i),
+    "nbk_fof_compress": ([_vp, _i64, _vp, _vp, _vp], _i),
+    "nbk_fof_minid": ([_vp, _i64, _vp, _i64, _vp, _vp, _vp], _i),
+    "nbk_fof_reduce": ([_i, _vp, _i64, _vp, _i64, _vp, _i, _i, _vp, _pd, _vp, _vp, _i64, _vp, _vp, _vp, _vp], _i),
     "nbk_fill": ([_vp, _i, _i64, _d, _vp], _i),
     "nbk_scale": ([_vp, _i, _i64, _d, _vp], _i),
     "nbk_axpy": ([_vp, _vp, _i, _i64, _d, _vp], _i),

@@ -1,9 +1,10 @@
 from .fftpower import FFTPower, FFTBase, ProjectedFFTPower, project_to_basis
 from .fftcorr import FFTCorr
 from .fftrecon import FFTRecon
+from .fof import FOF
 from .convpower import ConvolvedFFTPower, FKPCatalog, FKPWeightFromNbar, FKPCatalogMesh
 
 FKPPower = ConvolvedFFTPower
 
-__all__ = ['FFTCorr', 'FFTRecon', 'FFTPower', 'ProjectedFFTPower', 'FFTBase', 'project_to_basis', 'ConvolvedFFTPower', 'FKPPower', 'FKPCatalog',
+__all__ = ['FFTCorr', 'FOF', 'FFTRecon', 'FFTPower', 'ProjectedFFTPower', 'FFTBase', 'project_to_basis', 'ConvolvedFFTPower', 'FKPPower', 'FKPCatalog',
            'FKPWeightFromNbar', 'FKPCatalogMesh']

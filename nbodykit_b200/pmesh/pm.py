@@ -181,14 +181,20 @@ class SlabLayout(object):
             return rpos, rmass, sidx
         return rpos, rmass
 
-    def gather_back(self, values, sidx, out):
+    def gather_back(self, values, sidx, out, mode="sum"):
         """reverse of `route` for per-row results: `values[k]` was computed by the destination for the k-th row it
-        received; they travel back and are ADDED to out[source row] (pmesh `layout.gather(mode='sum')`)"""
+        received; they travel back and are combined into out[source row]: ADDED with mode='sum' (pmesh
+        `layout.gather(mode='sum')`), or the minimum kept with mode='min' (`layout.gather(mode=numpy.fmin)`)"""
+        if mode not in ("sum", "min"):
+            raise ValueError("gather_back: mode must be 'sum' or 'min', not %r" % (mode,))
         nsend = int(sum(self.sendcounts))
         back = torch.empty(nsend, dtype=values.dtype, device=values.device)
         self.comm.all_to_all_single(back, values.contiguous(), list(self.sendcounts), list(self.recvcounts))
         if nsend:
-            out.index_add_(0, sidx, back.to(out.dtype))
+            if mode == "sum":
+                out.index_add_(0, sidx, back.to(out.dtype))
+            else:
+                out.index_reduce_(0, sidx, back.to(out.dtype), "amin")
         return out
 
     def exchange(self, data):
