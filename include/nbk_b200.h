@@ -342,6 +342,45 @@ int nbk_fof_reduce(int op, const int64_t *label, int64_t n, const int32_t *order
                    int val_dtype, int dim, const int64_t *anchor, const double *box_host, const double *peak,
                    const int64_t *peakmax, int64_t ngroups, double *osum, int64_t *okey, int64_t *ocount, void *stream);
 
+/* Pair counts in a simulation box (SimulationBoxPairCount, algorithms/pair_counters/simbox.py; Corrfunc theory DD,
+ * DDsmu, DDrppi).  Both catalogues are bucketed on ONE cell grid, planned from (n2, r_max, box_host | lo_host,
+ * hi_host): cells of side >= r_max / 2, at most max(125, 2 n2) of them (the side grows when the cap binds).  A NULL box
+ * means non-periodic, and then lo/hi (the joint data bounds of both catalogues) place the grid.  r_max is the largest
+ * edge, or sqrt(rp_max^2 + pimax^2) in projected mode.  0 <= n <= 2^31-1.  Every call checks its arguments before any
+ * CUDA call.  The call sequence is workspace -> bucket (once per catalogue, or per chunk of primaries) -> count:
+ *   nbk_pc_workspace : bytes of scratch nbk_pc_bucket needs for n rows on that grid; ncell_host (optional, host
+ *                      int64[3]) receives the grid.  Negative on a rejected argument.
+ *   nbk_pc_stencil   : the neighbour offsets a cell visits, packed (ox+2)*25 + (oy+2)*5 + (oz+2), written to host
+ *                      int32[125]: every offset of the 5x5x5 block whose cell comes closer than r_max, each cell once
+ *                      when a periodic axis has fewer than 5 cells.  Returns how many (or a negative error).
+ *   nbk_pc_bucket    : counting sort of one catalogue.  pos [n][3] of pos_dtype F4|F8, w [n] of w_dtype F4|F8.
+ *                      spos: f64 [3][n] positions in cell order (wrapped into [0, L] when periodic), sw: f64 [n]
+ *                      weights, scell: int32 [n] cell of every slot, cstart: int32 [C+1] cell starts.
+ *   nbk_pc_count     : every ordered pair (primary slot, secondary slot) -> bin, ADDED to npairs uint64[nbins],
+ *                      wnpairs f64[nbins] (sum of w1 w2) and sepsum f64[nbins] (sum of r, or r_p in projected mode).
+ *                      Separations are float64, minimum image per axis when periodic; a pair counts when
+ *                      edges[k]^2 <= d^2 < edges[k+1]^2 (edges host f64, 2 <= nedges <= 1025, edges[0] > 0, increasing).
+ *                      mode NBK_PC_1D: nbins = nedges-1.  NBK_PC_2D: mu = |d_los| / d, pairs with mu >= 1 dropped,
+ *                      bin (k, min(floor(mu nmu), nmu-1)), nbins = (nedges-1) nmu.  NBK_PC_PROJECTED: r_p over the two
+ *                      axes other than los, pi = |d_los| < pimax (>= 1), npi = floor(pimax), bin (k, min(floor(pi npi /
+ *                      pimax), npi-1)).  los in 0..2.  rmax: the r_max the buckets were planned with, at least the
+ *                      largest separation a counted pair can have. */
+#define NBK_PC_1D 0
+#define NBK_PC_2D 1
+#define NBK_PC_PROJECTED 2
+int64_t nbk_pc_workspace(int64_t n, int64_t n2, double rmax, const double *box_host, const double *lo_host,
+                         const double *hi_host, int64_t *ncell_host);
+int nbk_pc_stencil(int64_t n2, double rmax, const double *box_host, const double *lo_host, const double *hi_host,
+                   int32_t *offsets_host);
+int nbk_pc_bucket(const void *pos, int pos_dtype, const void *w, int w_dtype, int64_t n, int64_t n2, double rmax,
+                  const double *box_host, const double *lo_host, const double *hi_host, void *work, int64_t work_bytes,
+                  double *spos, double *sw, int32_t *scell, int32_t *cstart, void *stream);
+int nbk_pc_count(int mode, const double *edges_host, int nedges, int nmu, double pimax, int los, double rmax,
+                 const double *spos1,
+                 const double *sw1, const int32_t *scell1, const int32_t *cstart1, int64_t n1, const double *spos2,
+                 const double *sw2, const int32_t *cstart2, int64_t n2, const double *box_host, const double *lo_host,
+                 const double *hi_host, uint64_t *npairs, double *wnpairs, double *sepsum, void *stream);
+
 /* elementwise helpers behind RealField/ComplexField `[...] = v`, `*= a`, `+= other`
  * (source/mesh/catalog.py:203,354,396-398; fftpower.py:128).  n counts REAL scalars. */
 int nbk_fill(void *x, int dtype, int64_t n, double value, void *stream);

@@ -13,7 +13,8 @@ CSRC = os.path.join(HERE, "csrc")
 OBJDIR = os.path.join(CSRC, "build")
 LIB = os.path.join(CSRC, "libnbk_b200.so")
 
-# (source, extra flags).  paint/binning carry bit-exact index arithmetic: no FMA contraction there.
+# (source, extra flags).  paint/binning carry bit-exact index arithmetic, and paircount bins float64 separations that
+# must equal the CPU oracle's: no FMA contraction there.
 SOURCES = [
     ("core.cu", []),
     ("paint.cu", ["--fmad=false"]),
@@ -23,6 +24,7 @@ SOURCES = [
     ("ylm.cu", []),
     ("route.cu", ["--fmad=false"]),
     ("fof.cu", []),
+    ("paircount.cu", ["--fmad=false"]),
 ]
 COMMON = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
           "-Xcompiler", "-fPIC", "-Xcompiler", "-O3"]
@@ -38,6 +40,7 @@ def _nvcc():
 def _stamp(path, flags):
     h = hashlib.sha1()
     for dep in [path, os.path.join(CSRC, "common.cuh"), os.path.join(CSRC, "fft_common.cuh"),
+                os.path.join(CSRC, "cellscan.cuh"),
                 os.path.join(CSRC, "ylm_table.inc"),
                 os.path.join(HERE, "..", "include", "nbk_b200.h")]:
         with open(dep, "rb") as f:

@@ -81,6 +81,11 @@ SIGNATURES = {
     "nbk_fof_compress": ([_vp, _i64, _vp, _vp, _vp], _i),
     "nbk_fof_minid": ([_vp, _i64, _vp, _i64, _vp, _vp, _vp], _i),
     "nbk_fof_reduce": ([_i, _vp, _i64, _vp, _i64, _vp, _i, _i, _vp, _pd, _vp, _vp, _i64, _vp, _vp, _vp, _vp], _i),
+    "nbk_pc_workspace": ([_i64, _i64, _d, _pd, _pd, _pd, _pi64], _i64),
+    "nbk_pc_stencil": ([_i64, _d, _pd, _pd, _pd, _vp], _i),
+    "nbk_pc_bucket": ([_vp, _i, _vp, _i, _i64, _i64, _d, _pd, _pd, _pd, _vp, _i64, _vp, _vp, _vp, _vp, _vp], _i),
+    "nbk_pc_count": ([_i, _pd, _i, _i, _d, _i, _d, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _i64, _pd, _pd, _pd,
+                      _vp, _vp, _vp, _vp], _i),
     "nbk_fill": ([_vp, _i, _i64, _d, _vp], _i),
     "nbk_scale": ([_vp, _i, _i64, _d, _vp], _i),
     "nbk_axpy": ([_vp, _vp, _i, _i64, _d, _vp], _i),

@@ -6,10 +6,9 @@
 //   nbk_fof_compress  : path compression -> component root of every row
 //   nbk_fof_minid     : component minimum of a per-row int64 value (per-root atomicMin, then a broadcast)
 //   nbk_fof_reduce    : dense per-group count / sum (optionally of periodically wrapped differences) / min / max
-#include "common.cuh"
+#include "cellscan.cuh"
 
 #define FOF_BLOCK 256
-#define FOF_SEG 4096            // elements per CTA of the offset scan (1024 threads x 4)
 
 struct FofGrid {
     int nc[3];                  // cells per axis
@@ -64,7 +63,7 @@ static inline int64_t fof_ncell(const FofGrid &g) { return (int64_t)g.nc[0] * g.
 
 // scratch: cell of every row int32[n] | counts / scatter cursors int32[C] | cell starts int32[C+1] | scan totals
 static int64_t fof_work_bytes(int64_t n, const FofGrid &g) {
-    int64_t C = fof_ncell(g), nseg = (C + 1 + FOF_SEG - 1) / FOF_SEG;
+    int64_t C = fof_ncell(g), nseg = nbk_scan_nseg(C);
     return (int64_t)(fof_align(4 * (size_t)n) + fof_align(4 * (size_t)C) + fof_align(4 * (size_t)(C + 1)) +
                      fof_align(4 * (size_t)(nseg + 1)));
 }
@@ -108,82 +107,6 @@ k_fof_cell(const T *__restrict__ pos, int n, FofGrid g, int *__restrict__ cell, 
         cell[i] = c;
         atomicAdd(&cnt[c], 1);
     }
-}
-
-// exclusive scan of cnt[0..C) into cstart[0..C], in three launches: segment totals, one CTA scanning the totals, then
-// every segment scans itself from its carry
-__global__ void __launch_bounds__(1024) k_fof_seg_totals(const int *__restrict__ cnt, int64_t C, int *__restrict__ segtot) {
-    __shared__ int wt[32];
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int64_t i = (int64_t)blockIdx.x * FOF_SEG + threadIdx.x * 4;
-    int s = 0;
-#pragma unroll
-    for (int j = 0; j < 4; j++) if (i + j < C) s += cnt[i + j];
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-    if (lane == 0) wt[wid] = s;
-    __syncthreads();
-    if (wid == 0) {
-        int x = wt[lane];
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
-        if (lane == 0) segtot[blockIdx.x] = x;
-    }
-}
-
-__device__ __forceinline__ int block_excl_scan(int v, int *wt, int *total) {
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    int inc = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        int nn = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += nn;
-    }
-    if (lane == 31) wt[wid] = inc;
-    __syncthreads();
-    if (wid == 0) {
-        int x = wt[lane];
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            int nn = __shfl_up_sync(0xffffffffu, x, o);
-            if (lane >= o) x += nn;
-        }
-        wt[lane] = x;
-    }
-    __syncthreads();
-    int r = (wid ? wt[wid - 1] : 0) + inc - v;
-    *total = wt[31];
-    __syncthreads();
-    return r;
-}
-
-__global__ void __launch_bounds__(1024) k_fof_scan_totals(int *__restrict__ segtot, int nseg) {
-    __shared__ int wt[32];
-    int carry = 0;
-    for (int base = 0; base < nseg; base += 1024) {
-        int i = base + threadIdx.x;
-        int v = i < nseg ? segtot[i] : 0, tot;
-        int e = block_excl_scan(v, wt, &tot);
-        if (i < nseg) segtot[i] = carry + e;
-        carry += tot;
-    }
-}
-
-__global__ void __launch_bounds__(1024)
-k_fof_seg_scan(const int *__restrict__ cnt, int64_t C, const int *__restrict__ segtot, int *__restrict__ cstart, int n) {
-    __shared__ int wt[32];
-    const int64_t i = (int64_t)blockIdx.x * FOF_SEG + threadIdx.x * 4;
-    int v[4];
-#pragma unroll
-    for (int j = 0; j < 4; j++) v[j] = (i + j < C) ? cnt[i + j] : 0;
-    int tot;
-    int run = segtot[blockIdx.x] + block_excl_scan(v[0] + v[1] + v[2] + v[3], wt, &tot);
-#pragma unroll
-    for (int j = 0; j < 4; j++) {
-        if (i + j < C) cstart[i + j] = run;
-        run += v[j];
-    }
-    if (blockIdx.x == 0 && threadIdx.x == 0) cstart[C] = n;
 }
 
 template <typename T>
@@ -440,19 +363,14 @@ extern "C" int nbk_fof_bucket(const void *pos, int dtype, int64_t n, double ll, 
     NBK_CHECK_ARG(pos && work && order && spos, "nbk_fof_bucket: null buffer");
     cudaStream_t s = (cudaStream_t)stream;
     const int64_t C = fof_ncell(g);
-    const int nseg = (int)((C + 1 + FOF_SEG - 1) / FOF_SEG);
     FofWork w = fof_carve(work, n, g);
     const int ni = (int)n, grid = nbk_grid_for(n, FOF_BLOCK, 8);
     NBK_CUDA(cudaMemsetAsync(w.cnt, 0, 4 * (size_t)C, s));
     if (dtype == NBK_F4) k_fof_cell<float><<<grid, FOF_BLOCK, 0, s>>>((const float *)pos, ni, g, w.cell, w.cnt);
     else k_fof_cell<double><<<grid, FOF_BLOCK, 0, s>>>((const double *)pos, ni, g, w.cell, w.cnt);
     NBK_LAUNCHED();
-    k_fof_seg_totals<<<nseg, 1024, 0, s>>>(w.cnt, C, w.segtot);
-    NBK_LAUNCHED();
-    k_fof_scan_totals<<<1, 1024, 0, s>>>(w.segtot, nseg);
-    NBK_LAUNCHED();
-    k_fof_seg_scan<<<nseg, 1024, 0, s>>>(w.cnt, C, w.segtot, w.cstart, ni);
-    NBK_LAUNCHED();
+    rc = nbk_cell_scan(w.cnt, C, w.segtot, w.cstart, ni, s);
+    if (rc != NBK_OK) return rc;
     NBK_CUDA(cudaMemsetAsync(w.cnt, 0, 4 * (size_t)C, s));
     if (dtype == NBK_F4) k_fof_scatter<float><<<grid, FOF_BLOCK, 0, s>>>((const float *)pos, ni, w.cell, w.cstart, w.cnt, order, (float *)spos);
     else k_fof_scatter<double><<<grid, FOF_BLOCK, 0, s>>>((const double *)pos, ni, w.cell, w.cstart, w.cnt, order, (double *)spos);
